@@ -17,10 +17,12 @@ peer memory per step (CLSTM_B200_DP=nccl selects ncclAllReduce + update instead)
            bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference --gpus 1 --steps 3 --warmup 1     # the reference's CPU path (oracle port)
 
-Prints ONE JSON line (rank 0).  Timing: every iteration is bracketed by CUDA events on the handle's stream, L2 is flushed
-in between; a reported step is the MEDIAN over steps x inner iterations of the per-iteration maximum over ranks (the mean
-and the full list are in the line as well).  `value` = whole-job px/s with the batch resident in HBM; `e2e` = the same
-through the input pipeline with pinned host buffers (H2D of the lines, D2H of the decoded result inside the timed region);
+Prints ONE JSON line (rank 0).  Timing: --steps training steps are timed, each bracketed by CUDA events on the handle's
+stream, L2 is flushed in between; the reported step is the MEDIAN over the steps of the per-step maximum over ranks (the
+mean and the full list are in the line as well).  --dump-outputs DIR writes what the last timed step returned (see
+dump_outputs) so that two builds can be compared output for output on identical seeded inputs.
+`value` = whole-job px/s with the batch resident in HBM; `e2e` = the same through the input pipeline with pinned host
+buffers (H2D of the lines, D2H of the decoded result inside the timed region);
 `roofline` for the dominant kernel from live CUDA-event phase timings; `cpu_baseline` = the CPU oracle port timed on this
 box's host cores on a bounded sample.
 """
@@ -63,7 +65,8 @@ def parse():
     ap.add_argument("--split", action="store_true", default=None,
                     help="--batch is the GLOBAL minibatch, split over the ranks (strong scaling)")
     ap.add_argument("--nclasses", type=int, default=83)
-    ap.add_argument("--inner", type=int, default=0, help="timed iterations per reported step (0: auto, ~20 ms per step)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the results of the last timed step as DIR/<name>.npy (float32, at most 64 MB in all)")
     ap.add_argument("--cpu-seconds", type=float, default=12.0, help="budget of the cpu_baseline sample")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the normalizer leg and the synchronous e2e form")
@@ -153,6 +156,29 @@ def make_batch(a, rank, world=1):
     xs = np.concatenate([x[offs[b]:offs[b + 1]] for b in mine], 0)
     labs = np.concatenate([labels[loffs[b]:loffs[b + 1]] for b in mine])
     return np.ascontiguousarray(xs), T[mine].copy(), labs.astype(np.int32), L[mine].copy()
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(d, net, mpl):
+    """What a caller of the timed step receives after it (rank 0): the decoded transcripts (clstm_b200_fetch_decoded,
+    classes and column locations per line, padded with -1), the updated weights and the momentum buffer, as float32
+    DIR/<name>.npy.  An array above its share of DUMP_BYTES is replaced by a sample of its elements at seeded positions
+    (the same for the same arguments)."""
+    dec = net.fetch_decoded(mpl)
+    cls = np.full((len(dec), mpl), -1, np.float32)
+    locs = np.full((len(dec), mpl), -1, np.float32)
+    for b, (c, l) in enumerate(dec):
+        cls[b, :len(c)] = c
+        locs[b, :len(l)] = l
+    outs = {"decoded_classes": cls, "decoded_locations": locs, "params": net.get_params(), "momentum": net.get_derivs()}
+    os.makedirs(d, exist_ok=True)
+    cap = DUMP_BYTES // len(outs) // 4
+    for name, v in outs.items():
+        if v.size > cap:
+            v = v.ravel()[np.sort(np.random.default_rng(0).choice(v.size, cap, replace=False))]
+        np.save(os.path.join(d, name + ".npy"), v)
 
 
 # ------------------------------------------------------------------------------------------ reference arm (CPU)
@@ -342,11 +368,10 @@ def run_b200(a):
     net.upload_batch(hx, T, labels, L)
     step_res = lambda: net.step_resident(LR, MOM, CLIP)  # noqa: E731
     warm = max(3, a.warmup)
-    est = float(np.median(timed(step_res, warm)))         # warm-up, also calibrates the inner iteration count
+    timed(step_res, warm)                                 # warm-up
     if dp_mode == "p2p-fused":
         net.peer_stats()                                  # arm the in-kernel counters of the fused all-reduce + update
-    inner = a.inner if a.inner > 0 else int(min(10, max(1, round(20.0 / max(est, 1e-3)))))
-    iters = a.steps * inner
+    iters = a.steps
     net.synchronize()
     barrier()
     t0 = time.time()
@@ -357,6 +382,9 @@ def run_b200(a):
     ms_step = float(np.median(ms_it))
     value = px_per_step / (ms_step / 1000.0)
     peer = net.peer_stats() if dp_mode == "p2p-fused" else None
+    mpl = int(T.max()) // 2 + 1
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, net, mpl)
     # second pass with per-phase CUDA events for the kernel table / roofline (everything on one stream)
     net.profile(True)
     prof_iters = min(iters, max(3, a.steps))
@@ -369,8 +397,6 @@ def run_b200(a):
     #             stream (clstm_b200_prefetch_batch), then clstm_b200_fetch_decoded(i) reads the result back.
     #  sync     : clstm_b200_train_step per batch (upload, step, fetch; nothing overlaps)
     # Every timed iteration contains one full H2D of a batch and one D2H of a step's decoded result.
-    mpl = int(T.max()) // 2 + 1
-
     def pipe_fn():
         net.step_prefetched(LR, MOM, CLIP)          # batch i (staged during step i-1)
         net.prefetch_batch(hx, T, labels, L)        # H2D of batch i+1 overlaps the kernels of step i
@@ -498,8 +524,7 @@ def run_b200(a):
                       "lines_per_gpu": len(T), "global_lines": a.batch if a.split else a.batch * world,
                       "columns_per_gpu": N, "global_columns": int(px_per_step // 48),
                       "l2": "flushed between timed iterations (256 MiB memset)",
-                      "timing": "median over steps x inner = %d x %d iterations, each its own CUDA-event pair, per-iteration max over ranks" % (a.steps, inner),
-                      "inner": inner,
+                      "timing": "median over %d steps, each its own CUDA-event pair, per-step max over ranks" % a.steps,
                       "weights": "reference LCG init (negbiased, 0.01), seed 0.222", "lr": LR, "momentum": MOM,
                       "lstm_kernel": net.lstm_variant, "parallelism": "dp%d" % world,
                       "grad_exchange": dp_mode},

@@ -35,7 +35,7 @@ def main():
             cmd += ["-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node", str(a.gpus), "--master-addr", "127.0.0.1",
                     "--master-port", str(29500 + (nh + T) % 400)]
         cmd += [os.path.join(ROOT, "bench.py"), "--gpus", str(a.gpus), "--steps", str(a.steps), "--warmup", str(a.warmup),
-                "--nhidden", str(nh), "--batch", str(a.batch), "--T", str(T), "--Tmax", "0", "--inner", "1", "--no-extras",
+                "--nhidden", str(nh), "--batch", str(a.batch), "--T", str(T), "--Tmax", "0", "--no-extras",
                 "--no-cpu-baseline"]
         r = subprocess.run(cmd, capture_output=True, text=True, cwd=ROOT)
         line = [ln for ln in r.stdout.split("\n") if ln.startswith("{")]
